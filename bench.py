@@ -175,6 +175,7 @@ def run_b200(args):
     recs = [synthetic.SyntheticRecording(s, positions[s]) for s in range(S)]
 
     diag_step = os.environ.get("BM_STEP_DIAG", "")
+    last = {}                                          # --dump-outputs: the latest step's loss and estimate
 
     def make_batch(meg_d, subj_d, subj_h):
         return synthetic.SyntheticBatch(meg_d, subj_d, [recs[s] for s in subj_h])
@@ -189,6 +190,8 @@ def run_b200(args):
         if world > 1 and diag_step != "no_allreduce":      # (BM_STEP_DIAG: diagnostic only)
             distrib.sync_gradients(model.parameters())
         opt.step()
+        if args.dump_outputs:
+            last.update(loss=loss, estimate=est)
         return loss
 
     def barrier():
@@ -244,6 +247,8 @@ def run_b200(args):
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = ms_total / args.steps
     value = world * B / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:            # before the e2e steps below move the model on
+        dump_outputs(args.dump_outputs, last["loss"], last["estimate"], model)
 
     # ---- end to end through the public API with HOST buffers (`e2e`) ------------------------------------
     # every step copies its inputs from pinned host memory (on a copy stream, one step ahead, like a DataLoader that
@@ -387,6 +392,36 @@ def run_b200(args):
         host_enqueue_ms_per_step=host_ms_value, step_ms=step_ms,
         clocks=clocks, e2e=e2e, gpu_launches=int(launches), roofline=roofline, cpu_baseline=cpu_baseline, also=also)
     emit(json.dumps(out))
+
+
+DUMP_ROWS = 8                  # segments of the estimate written by --dump-outputs
+DUMP_GRAD_MAX = 1 << 20        # entries of one gradient written in full; a larger one is sampled down to this many
+
+
+def dump_outputs(out_dir, loss, est, model):
+    """What one training step hands its caller, as float32 .npy files under `out_dir`: `loss`, `estimate` (DUMP_ROWS
+    segments of the [B, F, T] estimate) and `grad.<parameter>` (flattened; beyond DUMP_GRAD_MAX entries, that many of
+    them in ascending order).  Rows and entries are drawn by generators with fixed seeds, so that the same arguments write
+    the same selection and two builds can be compared file by file.  About 46 MB at cfg2, under 64 MB at every config."""
+    import zlib
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.randperm(est.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    arrays = {"loss": loss.detach().reshape(()), "estimate": est.detach()[rows.to(est.device)]}
+    for name, p in model.named_parameters():
+        if p.grad is None:
+            continue
+        g = p.grad.detach().reshape(-1)
+        if g.numel() > DUMP_GRAD_MAX:
+            gen = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            g = g[torch.randperm(g.numel(), generator=gen)[:DUMP_GRAD_MAX].sort().values.to(g.device)]
+        arrays["grad." + name] = g
+    total = 0
+    for name, a in arrays.items():
+        a = a.float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, f"--dump-outputs wrote {total / 2**20:.1f} MiB"
 
 
 def also_measured(cfg, model, clip, make_batch, resident, host, n_host, mask, dev, B, iters=5):
@@ -771,7 +806,11 @@ def main():
     ap.add_argument("--next-rows", action="store_true",
                     help="instead of the headline step: the SURVEY 8(f) rows (batch preparation, retrieval evaluation, "
                          "DeepMel), each beside a bounded CPU sample of its oracle; one GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last one's loss, estimate and gradients to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.next_rows):
+        ap.error("--dump-outputs applies to the B200 training step")
     if args.next_rows:
         from profiles import bench_next_rows      # its CPU legs are this file's cpu_baseline leg for those rows
         bench_next_rows.main(emit=emit)

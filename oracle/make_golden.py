@@ -10,11 +10,16 @@ the step (`bn.<key>`).  Everything fp32, produced by the reference's own code pa
     estimate = SimpleConv(...)(dict(meg=meg), batch)            simpleconv.py:198
     loss     = ClipLoss()(estimate, candidates, mask)           losses.py:104
     loss.backward()                                             solver.py:385
+The fixtures of `run_fresh` / `run_train_forward` keep them smaller: a digest of the initial state instead of the state,
+and a fixed sample of each larger gradient (`_model_case`); `seeded_init.json` holds per-tensor digests only.
 """
 from __future__ import annotations
 
+import hashlib
+import json
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
@@ -318,6 +323,175 @@ def run_ablation(name, change):
     print(f"{name}: loss={loss.item():.6f} est.std={est.std().item():.4f} params={sum(v.numel() for v in state.values())}")
 
 
+GRAD_SAMPLE = 256
+
+
+def tensor_sha256(t) -> str:
+    return hashlib.sha256(np.ascontiguousarray(t.detach().cpu().numpy()).tobytes()).hexdigest()
+
+
+def state_sha256(state) -> str:
+    """One digest over the keys, shapes, dtypes and bytes of a state_dict, in its order."""
+    h = hashlib.sha256()
+    for k, v in state.items():
+        h.update(f"{k} {tuple(v.shape)} {v.dtype} {tensor_sha256(v)}\n".encode())
+    return h.hexdigest()
+
+
+def grad_sample(key: str, numel: int) -> np.ndarray:
+    """The flat entries of parameter `key`'s gradient a fixture keeps: all of them up to GRAD_SAMPLE, else a fixed
+    sample of GRAD_SAMPLE (seeded by the name; numpy's legacy RandomState stream does not change between versions)."""
+    if numel <= GRAD_SAMPLE:
+        return np.arange(numel)
+    return np.sort(np.random.RandomState(zlib.crc32(key.encode())).choice(numel, GRAD_SAMPLE, replace=False))
+
+
+def seeded_state(cfg, seed, sha256):
+    """The initial clip_conv state_dict of the package's SimpleConv under torch.manual_seed(seed), checked against the
+    digest of the reference's (`sha256`: the raw bytes a `_model_case` fixture stores)."""
+    import brainmagick_b200 as bb
+    torch.manual_seed(seed)
+    model = bb.SimpleConv(in_channels=dict(meg=cfg.in_channels), out_channels=cfg.out_channels, n_subjects=cfg.n_subjects,
+                          **ref_loader.clip_conv_kwargs(hidden=cfg.hidden, depth=cfg.depth, merger_channels=cfg.merger_channels,
+                                                        initial_linear=cfg.initial_linear, merger_pos_dim=cfg.merger_pos_dim))
+    state = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    assert state_sha256(state) == bytes(np.asarray(sha256, dtype=np.uint8)).hex(), \
+        "the seeded initial state is not the reference's"
+    return state
+
+
+def _model_case(cfg, meg, cand, subj, pos, ban, est, loss, state, params=()):
+    """A fixture in the layout of `run_case` (readable by tests/conftest.load_golden) that holds the digest of the
+    reference's initial state instead of the state itself: the package's SimpleConv rebuilds it bit for bit from the same
+    seed (tests/test_boundary.py).  Gradients of `params`: the `grad_sample` entries and the norm of the whole."""
+    out = dict(cfg=np.array(cfg, dtype=np.int64), meg=meg.numpy(), candidates=cand.numpy(), subject_index=subj.numpy(),
+               rec_positions=pos.numpy(), rec_of_sample=subj.numpy(), ban_centre=ban.numpy(),
+               estimate=est.detach().numpy(), loss=loss.detach().numpy(),
+               state_sha256=np.frombuffer(bytes.fromhex(state_sha256(state)), dtype=np.uint8))
+    for k, v in params:
+        if v.grad is not None:
+            out["g." + k] = v.grad.numpy().ravel()[grad_sample(k, v.grad.numel())]
+            out["gnorm." + k] = np.float64(v.grad.double().norm())
+    return out
+
+
+FRESH_CASES = {"fresh_train": dict(seed=501, train=True), "fresh_eval": dict(seed=502, train=False)}
+
+
+def run_fresh(name, c):
+    """A depth-10 clip_conv with partly valid recordings, neither BN-perturbed nor shaped like the CASES: the
+    reference's estimate, loss and parameter gradients after one forward/backward in train or eval mode."""
+    seed, train = c["seed"], c["train"]
+    common, simpleconv, losses = ref_loader.load_reference()
+    torch.manual_seed(seed)
+    B, C, T, F, S, hidden, MC, IL, P = 7, 13, 41, 9, 4, 24, 16, 20, 72
+    kw = ref_loader.clip_conv_kwargs(hidden=hidden, depth=10, merger_channels=MC, initial_linear=IL, merger_pos_dim=P)
+    model = simpleconv.SimpleConv(in_channels=dict(meg=C), out_channels=F, n_subjects=S, **kw)
+    state = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    meg = torch.randn(B, C, T).clamp_(-20, 20)
+    cand = torch.randn(B + 3, F, T)
+    subj = torch.randint(0, S, (B,))
+    n_valid = [13, 9, 13, 6]
+    recs = [ref_loader.FakeRecording(s, C, n_valid[s], seed=seed) for s in range(S)]
+    for b in range(B):
+        meg[b, n_valid[int(subj[b])]:] = 0
+    batch = ref_loader.FakeBatch(meg, subj, [recs[int(s)] for s in subj])
+    pos = torch.full((S, C, 2), common.PositionGetter.INVALID)
+    for s in range(S):
+        lay = model.merger.position_getter.get_recording_layout(recs[s])
+        pos[s, :len(lay)] = lay
+    model.train(train)
+    torch.manual_seed(seed + 1)
+    ban = torch.rand(2)
+    torch.manual_seed(seed + 1)
+    est = model(dict(meg=meg.clone()), batch)
+    loss = losses.ClipLoss()(est, cand, torch.ones(B, 1, T, dtype=torch.bool))
+    loss.backward()
+    out = _model_case([B, B + 3, C, T, F, S, hidden, 10, MC, IL, P, int(train)], meg, cand, subj, pos, ban, est, loss,
+                      state, model.named_parameters())
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+    print(f"{name}: loss={loss.item():.6f} size={os.path.getsize(os.path.join(OUT, name + '.npz')) / 1024:.0f} KiB")
+
+
+def run_train_forward(name="train_forward"):
+    """A train-mode forward and loss at merger_pos_dim 128 with every channel valid (no backward)."""
+    common, simpleconv, losses = ref_loader.load_reference()
+    torch.manual_seed(1234)
+    C, F, S, T, B = 9, 6, 3, 31, 5
+    kw = ref_loader.clip_conv_kwargs(hidden=20, depth=10, merger_channels=8, initial_linear=12, merger_pos_dim=128)
+    model = simpleconv.SimpleConv(in_channels=dict(meg=C), out_channels=F, n_subjects=S, **kw)
+    state = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    meg, cand = torch.randn(B, C, T), torch.randn(B, F, T)
+    subj = torch.randint(0, S, (B,))
+    recs = [ref_loader.FakeRecording(s, C, seed=5) for s in range(S)]
+    batch = ref_loader.FakeBatch(meg, subj, [recs[int(s)] for s in subj])
+    pos = torch.stack([model.merger.position_getter.get_recording_layout(r) for r in recs])
+    model.train()
+    torch.manual_seed(7)
+    ban = torch.rand(2)
+    torch.manual_seed(7)
+    est = model(dict(meg=meg.clone()), batch)
+    loss = losses.ClipLoss()(est, cand, torch.ones(B, 1, T, dtype=torch.bool))
+    out = _model_case([B, B, C, T, F, S, 20, 10, 8, 12, 128, 1], meg, cand, subj, pos, ban, est, loss, state)
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+    print(f"{name}: loss={loss.item():.6f} size={os.path.getsize(os.path.join(OUT, name + '.npz')) / 1024:.0f} KiB")
+
+
+def run_prep_fresh(name="prep_fresh"):
+    """bm/norm.py ScaleReject (clip off and on) on scalers fitted to other data than prep_small's, per channel."""
+    norm = ref_loader.load_reference_norm()
+    torch.manual_seed(77)
+    B, C, T, off = 9, 8, 25, 2
+    fb = ref_loader.FakeFeaturesBuilder({"w": (4, True), "p": (3, False)})
+    scaler = norm.BatchScaler(fb, per_channel=True)
+    ids = [2, 3, 10]
+    for r in ids:
+        scaler.meg_scalers[r] = norm.RobustScaler().fit(torch.randn(300, C) * (1 + r))
+    feats_fit = torch.randn(40, fb.dimension, T)
+    for fname, fs in scaler.feature_scalers.items():
+        fs.fit(norm._as_nd(feats_fit[:, fb.get_slice(fname)]), norm._as_nd(torch.ones(40, 1, T, dtype=torch.bool)))
+    meg = torch.randn(B, C, T) * 40
+    rec = torch.tensor([2, 10, 3, 3, 2, 10, 10, 2, 3])
+    feats = torch.randn(B, fb.dimension, T)
+    mask = torch.ones(B, 1, T, dtype=torch.bool)
+    fc, fs_ = torch.zeros(fb.dimension), torch.ones(fb.dimension)
+    for fname, sc in scaler.feature_scalers.items():
+        if isinstance(sc, norm.StandardScaler):
+            fc[fb.get_slice(fname)], fs_[fb.get_slice(fname)] = sc.center_, sc.scale_
+    out = dict(rec_ids=np.array(ids), meg_center=np.stack([scaler.meg_scalers[r].center_.numpy() for r in ids]),
+               meg_scale=np.stack([scaler.meg_scalers[r].scale_.numpy() for r in ids]), feat_center=fc.numpy(),
+               feat_scale=fs_.numpy(), meg=meg.numpy(), recording_index=rec.numpy(), features=feats.numpy(),
+               features_mask=mask.numpy(), offset=np.int64(off), limit=np.float32(20.0))
+    for clip in (False, True):
+        sr = norm.ScaleReject(scaler, limit=20.0, clip=clip)
+        kept, keep = sr(ref_loader.FakeSegmentBatch(meg.clone(), feats.clone(), mask.clone(), rec.clone()))
+        out[f"clip{int(clip)}.keep"] = keep.numpy()
+        out[f"clip{int(clip)}.meg"] = kept.meg[..., off:].contiguous().numpy()
+        out[f"clip{int(clip)}.features"] = kept.features[..., :-off].contiguous().numpy()
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+    print(f"{name}: {len(out)} arrays, size={os.path.getsize(os.path.join(OUT, name + '.npz')) / 1024:.0f} KiB")
+
+
+SEEDED_INIT = dict(seed=77, C=30, F=17, S=5, hidden=48, MC=20, IL=24, P=128)
+
+
+def run_seeded_init(name="seeded_init"):
+    """The reference's freshly constructed clip_conv state_dict under torch.manual_seed (bm/train.py:76,109 model_hash)."""
+    c = SEEDED_INIT
+    _, simpleconv, _ = ref_loader.load_reference()
+    kw = dict(ref_loader.CLIP_CONV, hidden=dict(meg=c["hidden"]), merger_channels=c["MC"], initial_linear=c["IL"],
+              merger_pos_dim=c["P"])
+    torch.manual_seed(c["seed"])
+    model = simpleconv.SimpleConv(in_channels=dict(meg=c["C"]), out_channels=c["F"], n_subjects=c["S"], **kw)
+    out = dict(spec=c, subject_layers_repr=repr(model.subject_layers),
+               state=[dict(key=k, shape=list(v.shape), dtype=str(v.dtype), sha256=tensor_sha256(v))
+                      for k, v in model.state_dict().items()])
+    with open(os.path.join(OUT, name + ".json"), "w") as f:
+        json.dump(out, f, indent=1)
+        f.write("\n")
+    print(f"{name}: {len(out['state'])} tensors")
+
+
 if __name__ == "__main__":
     torch.set_num_threads(1)
     wanted = sys.argv[1:]
@@ -334,3 +508,9 @@ if __name__ == "__main__":
     for name, change in ABLATIONS.items():
         if not wanted or name in wanted:
             run_ablation(name, change)
+    for name, c in FRESH_CASES.items():
+        if not wanted or name in wanted:
+            run_fresh(name, c)
+    for name, fn in (("train_forward", run_train_forward), ("prep_fresh", run_prep_fresh), ("seeded_init", run_seeded_init)):
+        if not wanted or name in wanted:
+            fn(name)

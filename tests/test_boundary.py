@@ -1,14 +1,14 @@
 """CPU: the drop-in boundary -- constructor surface, state_dict layout, error behaviour, C-ABI symbols -- without
 any compute call (no GPU here)."""
 import ctypes
+import json
 import os
 import re
 
 import pytest
 import torch
 
-from conftest import GOLDEN_CASES, ROOT, load_golden
-from oracle import ref_loader
+from conftest import GOLDEN_CASES, GOLDEN_DIR, ROOT, load_golden
 
 CLIP_CONV = dict(hidden=dict(meg=320), batch_norm=True, depth=10, dilation_period=5, kernel_size=3, skip=True,
                  subject_layers=True, subject_dim=0, complex_out=True, glu=2, glu_context=1, merger=True,
@@ -60,23 +60,24 @@ def test_state_dict_layout_matches_reference(name):
     assert [n for n, _ in model.named_parameters()] == [k for k in ref if "running" not in k and "num_batches" not in k]
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present (GPU box)")
 def test_seeded_constructor_is_rng_identical_to_reference():
-    """same torch.manual_seed => bit-identical initial parameters (bm/train.py:76,109 model_hash)."""
+    """same torch.manual_seed => bit-identical initial parameters (bm/train.py:76,109 model_hash), against the digests of
+    the reference's state_dict (oracle/make_golden.py run_seeded_init)."""
     import brainmagick_b200 as bb
-    _, simpleconv, _ = ref_loader.load_reference()
-    kw = _kw(hidden=dict(meg=48), merger_channels=20, initial_linear=24, merger_pos_dim=128)
-    torch.manual_seed(77)
-    ref = simpleconv.SimpleConv(in_channels=dict(meg=30), out_channels=17, n_subjects=5,
-                                **{k: (dict(v) if isinstance(v, dict) else v) for k, v in kw.items()})
-    torch.manual_seed(77)
-    mine = bb.SimpleConv(in_channels=dict(meg=30), out_channels=17, n_subjects=5,
-                         **{k: (dict(v) if isinstance(v, dict) else v) for k, v in kw.items()})
-    rs, ms = ref.state_dict(), mine.state_dict()
-    assert list(rs) == list(ms)
-    for k in rs:
-        assert torch.equal(rs[k], ms[k]), k
-    assert repr(mine.subject_layers) == repr(ref.subject_layers)
+    from oracle import make_golden
+    with open(os.path.join(GOLDEN_DIR, "seeded_init.json")) as f:
+        ref = json.load(f)
+    c = ref["spec"]
+    assert c == make_golden.SEEDED_INIT
+    kw = _kw(hidden=dict(meg=c["hidden"]), merger_channels=c["MC"], initial_linear=c["IL"], merger_pos_dim=c["P"])
+    torch.manual_seed(c["seed"])
+    mine = bb.SimpleConv(in_channels=dict(meg=c["C"]), out_channels=c["F"], n_subjects=c["S"], **kw)
+    ms = mine.state_dict()
+    assert list(ms) == [e["key"] for e in ref["state"]]
+    for e in ref["state"]:
+        v = ms[e["key"]]
+        assert [list(v.shape), str(v.dtype), make_golden.tensor_sha256(v)] == [e["shape"], e["dtype"], e["sha256"]], e["key"]
+    assert repr(mine.subject_layers) == ref["subject_layers_repr"]
 
 
 def test_constructor_errors_and_unsupported_options():

@@ -1,11 +1,9 @@
 """CPU: pins the oracle restatement (oracle/bm_oracle.py) against the golden vectors produced by the verbatim
-reference modules (oracle/make_golden.py), and -- when /root/reference is present (build container only) --
-against the live reference at a second, freshly seeded configuration."""
-import pytest
+reference modules (oracle/make_golden.py), among them a second, separately seeded configuration (train_forward)."""
 import torch
 
-from oracle import bm_oracle, ref_loader
-from conftest import rel_err
+from oracle import bm_oracle, make_golden
+from conftest import load_golden, rel_err
 
 TOL = 2e-5   # fp32-vs-fp32 with different summation orders; the stated parity bar is 1e-4
 
@@ -52,31 +50,16 @@ def test_oracle_fp64_agrees_with_fp32(golden):
     assert rel_err(est64.float(), t["estimate"]) < 2e-5
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present (GPU box)")
 def test_oracle_matches_live_reference():
-    common, simpleconv, losses = ref_loader.load_reference()
-    torch.manual_seed(1234)
-    C, F, S, T, B = 9, 6, 3, 31, 5
-    kw = ref_loader.clip_conv_kwargs(hidden=20, depth=10, merger_channels=8, initial_linear=12, merger_pos_dim=128)
-    model = simpleconv.SimpleConv(in_channels=dict(meg=C), out_channels=F, n_subjects=S, **kw)
-    cfg = bm_oracle.Config(in_channels=C, out_channels=F, n_subjects=S, hidden=20, depth=10,
-                           merger_channels=8, initial_linear=12, merger_pos_dim=128)
-    assert cfg.dilations() == [1, 2, 4, 8, 16, 1, 2, 4, 8, 16]
-    meg, cand = torch.randn(B, C, T), torch.randn(B, F, T)
-    subj = torch.randint(0, S, (B,))
-    recs = [ref_loader.FakeRecording(s, C, seed=5) for s in range(S)]
-    batch = ref_loader.FakeBatch(meg, subj, [recs[int(s)] for s in subj])
-    pos = torch.stack([model.merger.position_getter.get_recording_layout(r) for r in recs])
-    model.train()
-    torch.manual_seed(7)
-    ban = torch.rand(2)
-    torch.manual_seed(7)
-    est = model(dict(meg=meg.clone()), batch)
-    loss = losses.ClipLoss()(est, cand, torch.ones(B, 1, T, dtype=torch.bool))
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    est_o = bm_oracle.simpleconv_forward(p, cfg, meg, pos, subj, subj, True, ban)
-    assert rel_err(est_o, est.detach()) < TOL
-    assert abs(bm_oracle.clip_loss(est_o, cand).item() - loss.item()) < 1e-5
+    """The reference's train-mode forward and loss at merger_pos_dim 128 (oracle/make_golden.py run_train_forward),
+    from its seeded initial state."""
+    cfg, train, t = load_golden("train_forward")
+    assert train and cfg.dilations() == [1, 2, 4, 8, 16, 1, 2, 4, 8, 16]
+    p = make_golden.seeded_state(cfg, 1234, t["state_sha256"])
+    subj = t["subject_index"]
+    est_o = bm_oracle.simpleconv_forward(p, cfg, t["meg"], t["rec_positions"], subj, subj, True, t["ban_centre"])
+    assert rel_err(est_o, t["estimate"]) < TOL
+    assert abs(bm_oracle.clip_loss(est_o, t["candidates"]).item() - t["loss"].item()) < 1e-5
 
 
 def test_synthetic_batch_shapes():

@@ -1,19 +1,18 @@
-"""Live pin of the oracles against the VERBATIM reference modules (loaded from /root/reference by `oracle/ref_loader.py`).
-Runs only where the reference tree exists (the build container); skipped on the GPU box, where the committed fixtures carry
-the pin.  Two things are checked: (1) the committed fixtures are exactly what the committed generator produces from the
-reference today; (2) on fresh inputs that no fixture holds, oracle == reference."""
+"""Pin of the oracles against the VERBATIM reference modules.  Two things are checked: (1) the committed fixtures are
+exactly what the committed generator produces from the reference today -- only where a brainmagick source tree is at hand
+(`oracle/ref_loader.py`, BM_REFERENCE_ROOT); (2) on inputs that no other fixture holds, oracle == reference, against what
+the reference computed on them (oracle/make_golden.py: fresh_train, fresh_eval, prep_fresh)."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN_DIR, rel_err
-from oracle import bm_oracle, prep_oracle, ref_loader
-
-pytestmark = pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
+from conftest import GOLDEN_DIR, load_arrays, load_golden, rel_err
+from oracle import bm_oracle, make_golden, prep_oracle, ref_loader
 
 
+@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs the brainmagick source tree (BM_REFERENCE_ROOT)")
 @pytest.mark.parametrize("kind,name", [("case", "train_depth4"), ("case", "eval_small"), ("prep", "prep_small"),
                                        ("retrieval", "retrieval_small"), ("deepmel", "deepmel_nobn"),
                                        ("ablation", "ablation_subject_embedding")])
@@ -45,72 +44,34 @@ def test_fixtures_are_reproducible_from_the_reference(kind, name, tmp_path, monk
 
 @pytest.mark.parametrize("seed,train", [(501, True), (502, False)])
 def test_oracle_equals_live_reference_on_fresh_inputs(seed, train):
-    common, simpleconv, losses = ref_loader.load_reference()
-    torch.manual_seed(seed)
-    B, C, T, F, S, hidden, MC, IL, P = 7, 13, 41, 9, 4, 24, 16, 20, 72
-    kw = ref_loader.clip_conv_kwargs(hidden=hidden, depth=10, merger_channels=MC, initial_linear=IL, merger_pos_dim=P)
-    model = simpleconv.SimpleConv(in_channels=dict(meg=C), out_channels=F, n_subjects=S, **kw)
-    state = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    meg = torch.randn(B, C, T).clamp_(-20, 20)
-    cand = torch.randn(B + 3, F, T)
-    subj = torch.randint(0, S, (B,))
-    n_valid = [13, 9, 13, 6]
-    recs = [ref_loader.FakeRecording(s, C, n_valid[s], seed=seed) for s in range(S)]
-    for b in range(B):
-        meg[b, n_valid[int(subj[b])]:] = 0
-    batch = ref_loader.FakeBatch(meg, subj, [recs[int(s)] for s in subj])
-    pos = torch.full((S, C, 2), common.PositionGetter.INVALID)
-    for s in range(S):
-        lay = model.merger.position_getter.get_recording_layout(recs[s])
-        pos[s, :len(lay)] = lay
-    model.train(train)
-    torch.manual_seed(seed + 1)
-    ban = torch.rand(2)
-    torch.manual_seed(seed + 1)
-    est = model(dict(meg=meg.clone()), batch)
-    loss = losses.ClipLoss()(est, cand, torch.ones(B, 1, T, dtype=torch.bool))
-    loss.backward()
-    cfg = bm_oracle.Config(in_channels=C, out_channels=F, n_subjects=S, hidden=hidden, merger_channels=MC,
-                           initial_linear=IL, merger_pos_dim=P)
-    ref = bm_oracle.training_step(state, cfg, meg, pos, subj, subj, cand, ban_centre=ban, training=train)
-    assert rel_err(ref["estimate"], est.detach()) < 2e-6
-    assert abs(float(ref["loss"]) - float(loss.detach())) < 1e-6
-    for name, p in model.named_parameters():
-        if p.grad is None:
-            continue
-        if p.grad.norm() < 1e-6:
-            assert ref["grads"][name].abs().max() < 1e-5, name
+    name = "fresh_train" if train else "fresh_eval"
+    assert make_golden.FRESH_CASES[name] == dict(seed=seed, train=train)
+    cfg, train_, t = load_golden(name)
+    assert train_ == train
+    state = make_golden.seeded_state(cfg, seed, t["state_sha256"])
+    subj = t["subject_index"]
+    ref = bm_oracle.training_step(state, cfg, t["meg"], t["rec_positions"], subj, subj, t["candidates"],
+                                  ban_centre=t["ban_centre"], training=train)
+    assert rel_err(ref["estimate"], t["estimate"]) < 2e-6
+    assert abs(float(ref["loss"]) - float(t["loss"])) < 1e-6
+    grads = [k[2:] for k in t if k.startswith("g.")]
+    assert grads and set(grads) <= set(ref["grads"])
+    for key in grads:                      # the reference's gradient at the fixture's `grad_sample` entries
+        g = ref["grads"][key].reshape(-1)[torch.from_numpy(make_golden.grad_sample(key, ref["grads"][key].numel()))]
+        if t["gnorm." + key] < 1e-6:
+            assert ref["grads"][key].abs().max() < 1e-5, key
         else:
-            assert rel_err(ref["grads"][name], p.grad) < 3e-5, name
+            assert rel_err(g, t["g." + key]) < 3e-5, key
 
 
 def test_prep_oracle_equals_live_reference_on_fresh_inputs():
-    norm = ref_loader.load_reference_norm()
-    torch.manual_seed(77)
-    B, C, T, off = 9, 8, 25, 2
-    fb = ref_loader.FakeFeaturesBuilder({"w": (4, True), "p": (3, False)})
-    scaler = norm.BatchScaler(fb, per_channel=True)
-    ids = [2, 3, 10]
-    for r in ids:
-        scaler.meg_scalers[r] = norm.RobustScaler().fit(torch.randn(300, C) * (1 + r))
-    feats_fit = torch.randn(40, fb.dimension, T)
-    for fname, fs in scaler.feature_scalers.items():
-        fs.fit(norm._as_nd(feats_fit[:, fb.get_slice(fname)]), norm._as_nd(torch.ones(40, 1, T, dtype=torch.bool)))
-    meg = torch.randn(B, C, T) * 40
-    rec = torch.tensor([2, 10, 3, 3, 2, 10, 10, 2, 3])
-    feats = torch.randn(B, fb.dimension, T)
-    mask = torch.ones(B, 1, T, dtype=torch.bool)
-    fc, fs_ = torch.zeros(fb.dimension), torch.ones(fb.dimension)
-    for fname, sc in scaler.feature_scalers.items():
-        if isinstance(sc, norm.StandardScaler):
-            fc[fb.get_slice(fname)], fs_[fb.get_slice(fname)] = sc.center_, sc.scale_
-    center = {r: scaler.meg_scalers[r].center_.numpy() for r in ids}
-    scale = {r: scaler.meg_scalers[r].scale_.numpy() for r in ids}
+    t = load_arrays("prep_fresh")
+    ids, off = [int(r) for r in t["rec_ids"]], int(t["offset"])
+    center = {r: t["meg_center"][i] for i, r in enumerate(ids)}
+    scale = {r: t["meg_scale"][i] for i, r in enumerate(ids)}
     for clip in (False, True):
-        sr = norm.ScaleReject(scaler, limit=20.0, clip=clip)
-        kept, keep = sr(ref_loader.FakeSegmentBatch(meg.clone(), feats.clone(), mask.clone(), rec.clone()))
-        got = prep_oracle.prepare(meg.numpy(), rec.numpy(), center, scale, feats.numpy(), mask.numpy(), fc.numpy(),
-                                  fs_.numpy(), limit=20.0, clip=clip, offset_samples=off)
-        assert np.array_equal(got["keep"], keep.numpy())
-        assert np.array_equal(got["meg"], kept.meg[..., off:].numpy())
-        assert np.array_equal(got["features"], kept.features[..., :-off].numpy())
+        got = prep_oracle.prepare(t["meg"], t["recording_index"], center, scale, t["features"], t["features_mask"],
+                                  t["feat_center"], t["feat_scale"], limit=float(t["limit"]), clip=clip, offset_samples=off)
+        assert np.array_equal(got["keep"], t[f"clip{int(clip)}.keep"])
+        assert np.array_equal(got["meg"], t[f"clip{int(clip)}.meg"])
+        assert np.array_equal(got["features"], t[f"clip{int(clip)}.features"])
