@@ -14,10 +14,10 @@ if "CUDA_DEVICE_MAX_CONNECTIONS" not in _os.environ and not _torch.cuda.is_initi
     _os.environ["CUDA_DEVICE_MAX_CONNECTIONS"] = "32"
 
 from .simpleconv import SimpleConv  # noqa: F401,E402
-from .losses import ClipLoss  # noqa: F401,E402
+from .losses import ClipLoss, L1Loss, L2Loss  # noqa: F401,E402
 from .common import ChannelMerger, ConvSequence, FourierEmb, PositionGetter, SubjectLayers  # noqa: F401
 from .features import DeepMel  # noqa: F401
 from .norm import BatchScaler, ScaleReject  # noqa: F401
 
-__all__ = ["SimpleConv", "ClipLoss", "ChannelMerger", "ConvSequence", "FourierEmb", "PositionGetter",
+__all__ = ["SimpleConv", "ClipLoss", "L1Loss", "L2Loss", "ChannelMerger", "ConvSequence", "FourierEmb", "PositionGetter",
            "SubjectLayers", "DeepMel", "BatchScaler", "ScaleReject"]

@@ -76,6 +76,8 @@ SIGNATURES = {
     "bm_scale_clamp_crop": [P, P, P, P, I, I, I, I, I, F, I, I, P, P, P],
     "bm_reject_compact": [P, P, L, F, I, P, P, P, P],
     "bm_gather_rows": [P, P, I, L, P, P],
+    "bm_regression_loss_fwd": [P, P, P, I, I, I, I, I, P, P, P],
+    "bm_regression_loss_bwd": [P, P, P, P, P, I, I, I, I, I, P, P, P],
     "bm_bn_act_skip_fwd": [P, P, P, P, P, P, P, L, I, I, F, P],
     "bm_bn_act_skip_bwd": [P, P, P, P, P, P, I, L, I, I, F, P, P, P, P, P],
     "bm_clip_loss_bwd_cand": [P, P, P, P, P, P, I, I, L, I, P, P, P, P, P],

@@ -15,6 +15,7 @@
 #include "retrieval.cuh"
 #include "prep.cuh"
 #include "convseq.cuh"
+#include "regression.cuh"
 
 namespace bm {
 thread_local char g_last_error[512] = "";
@@ -826,6 +827,44 @@ extern "C" int bm_gather_rows(const float* x, const int* rows, int n_rows, long 
                               bm_stream_t stream) {
     BM_CHECK_ARG(x && rows && y && n_rows > 0 && row_elems > 0);
     gather_rows_kernel<<<ew_grid((long long)n_rows * row_elems), 256, 0, ST(stream)>>>(x, rows, n_rows, row_elems, y);
+    BM_CHECK_LAUNCH();
+    return 0;
+}
+
+// =================================================================================================
+// Regression objectives (L1Loss / L2Loss, bm/losses.py:11-26)
+// =================================================================================================
+extern "C" int bm_regression_loss_fwd(const float* est, const float* out, const unsigned char* mask, int B, int F, int Fm,
+                                      int T, int p, double* workspace, float* loss, bm_stream_t stream) {
+    BM_CHECK_ARG(est && out && mask && workspace && loss);
+    BM_CHECK_ARG(B > 0 && F > 0 && T > 0 && (Fm == 1 || Fm == F) && (p == 1 || p == 2));
+    const long long rows = (long long)B * F;
+    const int grid = regression_grid(rows * T);
+    const bool vec = T % 4 == 0 && reg_aligned(est, 16) && reg_aligned(out, 16) && reg_aligned(mask, 4);
+    cudaStream_t st = ST(stream);
+    BM_CUDA(cudaMemsetAsync(workspace + REG_WS_TICKET, 0, sizeof(unsigned int), st));
+    if (p == 1)
+        launch_regression_fwd_p<1>(vec, grid, est, out, mask, rows, F, Fm == F, T, workspace, loss, st);
+    else
+        launch_regression_fwd_p<2>(vec, grid, est, out, mask, rows, F, Fm == F, T, workspace, loss, st);
+    BM_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int bm_regression_loss_bwd(const float* est, const float* out, const unsigned char* mask, const float* gout,
+                                      const double* workspace, int B, int F, int Fm, int T, int p, float* dest, float* dout,
+                                      bm_stream_t stream) {
+    BM_CHECK_ARG(est && out && mask && gout && workspace && (dest || dout));
+    BM_CHECK_ARG(B > 0 && F > 0 && T > 0 && (Fm == 1 || Fm == F) && (p == 1 || p == 2));
+    const long long rows = (long long)B * F;
+    const int grid = regression_grid(rows * T);
+    const bool vec = T % 4 == 0 && reg_aligned(est, 16) && reg_aligned(out, 16) && reg_aligned(mask, 4) &&
+                     reg_aligned(dest, 16) && reg_aligned(dout, 16);
+    cudaStream_t st = ST(stream);
+    if (p == 1)
+        launch_regression_bwd_p<1>(vec, grid, est, out, mask, rows, F, Fm == F, T, gout, workspace, dest, dout, st);
+    else
+        launch_regression_bwd_p<2>(vec, grid, est, out, mask, rows, F, Fm == F, T, gout, workspace, dest, dout, st);
     BM_CHECK_LAUNCH();
     return 0;
 }

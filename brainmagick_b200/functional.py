@@ -3,7 +3,8 @@
 `encoder_forward` is SimpleConv.forward at the clip_conv configuration (bm/models/simpleconv.py:198-249) as ONE
 autograd node: its backward launches the hand-written gradient kernels in reverse order, so `loss.backward()`
 leaves ordinary dense `.grad` tensors on every parameter (what bm/solver.py:384-387 and
-flashy.distrib.sync_model expect).  `clip_loss` / `clip_scores` are ClipLoss (bm/losses.py:77-114).
+flashy.distrib.sync_model expect).  `clip_loss` / `clip_scores` are ClipLoss (bm/losses.py:77-114);
+`regression_loss` is L1Loss / L2Loss (bm/losses.py:11-26).
 
 Kernel selection is by shape only: contractions whose channel counts fit the tcgen05 tiling (K % 32 == 0 and an
 N tile of 64..160 dividing N -- every layer of the real clip_conv model) run on the tensor-core kernels
@@ -1014,6 +1015,65 @@ class _ClipLossFn(torch.autograd.Function):
 
 def clip_loss(estimate, candidate, target_offset: int = 0):
     return _ClipLossFn.apply(estimate, candidate, target_offset)
+
+
+# ----------------------------------------------------------------------------------------------------
+# L1Loss / L2Loss (bm/losses.py:11-26): mean of |estimate - output|^p over mask.expand_as(estimate)
+# ----------------------------------------------------------------------------------------------------
+REGRESSION_WS_DOUBLES = 1186           # BM_REGRESSION_WS_DOUBLES of include/bm_b200.h
+
+
+def _regression_mask(mask: torch.Tensor, estimate: torch.Tensor) -> torch.Tensor:
+    """The selection the reference indexes with, `mask.expand_as(estimate)`, as contiguous bytes [B, 1, T] when it is the
+    same for every feature (the solver's features_mask), else [B, F, T]."""
+    full = mask.expand_as(estimate)
+    if full.stride(1) == 0:
+        full = full[:, :1]
+    return full.contiguous().view(torch.uint8)
+
+
+class _RegressionLossFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, estimate, output, mask, p: int):
+        est = estimate.contiguous()
+        out = output.contiguous()            # the solver's targets are a time-cropped view (features[..., :-offset])
+        m = _regression_mask(mask, est)
+        B, F, T = est.shape
+        ws = _empty((REGRESSION_WS_DOUBLES,), est, torch.float64)
+        loss = _empty((1,), est)
+        call("bm_regression_loss_fwd", ptr(est), ptr(out), ptr(m), B, F, m.shape[1], T, p, ptr(ws), ptr(loss), stream())
+        ctx.save_for_backward(est, out, m, ws)      # ws holds the selected count the backward reads
+        ctx.p = p
+        return loss.reshape(())
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, gout):
+        est, out, m, ws = ctx.saved_tensors
+        B, F, T = est.shape
+        dest = _empty(est.shape, est) if ctx.needs_input_grad[0] else None
+        dout = _empty(est.shape, est) if ctx.needs_input_grad[1] else None
+        g = gout.reshape(1).contiguous().float()
+        call("bm_regression_loss_bwd", ptr(est), ptr(out), ptr(m), ptr(g), ptr(ws), B, F, m.shape[1], T, ctx.p, ptr(dest),
+             ptr(dout), stream())
+        return dest, dout, None, None
+
+
+def regression_loss(estimate: torch.Tensor, output: torch.Tensor, mask: torch.Tensor, p: int) -> torch.Tensor:
+    """mean over the elements selected by `mask.expand_as(estimate)` of |estimate - output| (p = 1, nn.L1Loss) or
+    (estimate - output)^2 (p = 2, nn.MSELoss), as a 0-dim tensor; no host synchronisation.  estimate, output [B, F, T]
+    fp32; mask bool, broadcastable to [B, F, T] ([B, 1, T] in the solver)."""
+    if p not in (1, 2):
+        raise ValueError(f"p must be 1 or 2, got {p}")
+    if mask is None:
+        raise TypeError("a mask is required (bm/losses.py:13 expands it over the estimate)")
+    if mask.dtype != torch.bool:
+        raise TypeError(f"the mask selects elements and must be torch.bool, got {mask.dtype}")
+    if estimate.dim() != 3 or estimate.shape != output.shape:
+        raise ValueError(f"estimate {tuple(estimate.shape)} and output {tuple(output.shape)} must be the same [B, F, T]")
+    if not (estimate.device == output.device == mask.device):
+        raise ValueError(f"estimate on {estimate.device}, output on {output.device}, mask on {mask.device}")
+    return _RegressionLossFn.apply(estimate, output, mask, p)
 
 
 # ----------------------------------------------------------------------------------------------------

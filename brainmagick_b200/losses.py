@@ -8,6 +8,9 @@ the `linear` projection is constructed but never applied (losses.py:35,82), targ
 Extension (SURVEY.md 8(e), not in the reference): `global_negatives=True` all-gathers the candidates over the
 default process group before scoring, so every rank contrasts against the global batch; when the candidates require
 grad (a trainable feature model) the gather is differentiable (reduce-scatter of the candidate gradients).
+
+Drop-in `L1Loss` / `L2Loss` (reference: bm/losses.py:11-26, the solver's 'l1' and 'mse' objectives): no-argument
+constructor, `forward(estimate, output, mask)`; the masked mean and its gradient run in CUDA (`functional.regression_loss`).
 """
 from __future__ import annotations
 
@@ -15,8 +18,38 @@ import weakref
 
 import torch
 
+from . import common as CM
 from . import functional as BF
 from . import distrib
+
+
+class _MaskedLoss(torch.nn.Module):
+    """bm/losses.py:11-14: the mean of the per-element loss over `mask.expand_as(estimate)`, on one CUDA pass forward and
+    one backward (`functional.regression_loss`) instead of a boolean gather, which synchronises with the host."""
+    _p = 0
+
+    def forward(self, estimate, output, mask=None):
+        for name, t in (("estimate", estimate), ("output", output)):
+            CM._require_cuda_fp32(t, f"{type(self).__name__} ({name})")
+        return BF.regression_loss(estimate, output, mask, self._p)
+
+
+class L1Loss(_MaskedLoss):
+    """The solver's `optim.loss=l1` (bm/solver.py:76-94): mean |estimate - output| over the masked elements."""
+    _p = 1
+
+    def __init__(self):
+        super().__init__()
+        self._loss = torch.nn.L1Loss()           # never called; kept so that repr() and state_dict() match the reference
+
+
+class L2Loss(_MaskedLoss):
+    """The solver's `optim.loss=mse`: mean (estimate - output)^2 over the masked elements."""
+    _p = 2
+
+    def __init__(self):
+        super().__init__()
+        self._loss = torch.nn.MSELoss()          # never called; kept so that repr() and state_dict() match the reference
 
 
 class ClipLoss(torch.nn.Module):

@@ -233,6 +233,23 @@ int bm_reject_compact(const unsigned int* peak_bits, const unsigned char* mask, 
                       int B, unsigned char* keep, int* keep_rows, int* n_keep, bm_stream_t stream);
 int bm_gather_rows(const float* x, const int* rows, int n_rows, long long row_elems, float* y, bm_stream_t stream);
 
+/* ---- Regression objectives: L1Loss / L2Loss (bm/losses.py:11-26), the solver's 'l1' and 'mse' (bm/solver.py:76-94) -----
+ * loss = mean over the selected elements of |est - out|^p (p = 1 or 2), selected = mask.expand_as(est):
+ * est, out [B,F,T] fp32; mask [B,Fm,T] bytes (torch.bool: 0 / 1), Fm = 1 (one mask per sample and time, broadcast over F)
+ * or Fm = F.  Unselected elements are never used arithmetically (a NaN or inf there does not reach the loss or the
+ * gradient); an empty selection gives loss NaN (0/0) and zero gradients.
+ * workspace: BM_REGRESSION_WS_DOUBLES doubles of caller-owned scratch.  bm_regression_loss_fwd fills it with fp64 partial
+ * sums (reduced in a fixed order by the last block: the loss is bit-identical from call to call) and the selected count,
+ * which bm_regression_loss_bwd reads on the device, so keep the buffer unchanged until the backward.  loss [1] fp32.
+ * bm_regression_loss_bwd: dest = selected ? p |d|^(p-1) sign(d) gout / count : 0 with d = est - out (sign(0) = 0, NaN
+ * propagates); dout = -dest.  gout [1] is the incoming gradient on the device; dest or dout may be NULL (not both). */
+#define BM_REGRESSION_WS_DOUBLES 1186
+int bm_regression_loss_fwd(const float* est, const float* out, const unsigned char* mask, int B, int F, int Fm, int T,
+                           int p, double* workspace, float* loss, bm_stream_t stream);
+int bm_regression_loss_bwd(const float* est, const float* out, const unsigned char* mask, const float* gout,
+                           const double* workspace, int B, int F, int Fm, int T, int p, float* dest, float* dout,
+                           bm_stream_t stream);
+
 /* ---- tcgen05 (5th-gen tensor core) versions of K3/K4: 3xTF32 implicit-GEMM conv ---------------------------
  * Same arithmetic contract as bm_conv1d_fwd / bm_conv1d_bwd_data / bm_conv1d_glu_fwd (fp32-faithful: every
  * product is hi*hi + lo*hi + hi*lo of tf32 splits, fp32 accumulation in tensor memory).
